@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the FourierGrid / DVGO rendering hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|reference-gpu] [--workload truck|bicycle]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): ray-samples/sec, 8192 rays x 512 samples, one training iteration per step
 (forward + loss + backward + total-variation + MaskedAdam, i.e. run_train.py:251-288 of the reference).
@@ -22,6 +23,9 @@ A/B switches (env): UBN_BENCH_TAIL=peer|pipelined|sequential (training-step tail
 UBN_TV_IMPL=1|0 (streaming / element-per-thread TV; scripts/check_tv_stream.py), UBN_RGBNET_MODE=tc3|tc1|simt,
 UBN_RGBNET_BWD_MODE=fused|tc3|simt (every mode is exercised by tests/test_gpu_models.py::test_fused_rgbnet_vs_torch),
 UBN_NCCL_HIGH_PRIORITY=1|0, UBN_PEER_MAP=auto|symm|ipc.
+`--dump-outputs DIR` (rank 0): after the timed steps, what the last timed step computed -- the returned arrays of the model
+forward and the loss (training workloads) or the frame (render workloads), and the parameters after its update -- as
+DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs (dump_outputs).
 """
 import argparse
 import json
@@ -39,6 +43,37 @@ import torch  # noqa: E402
 
 N_RAYS, N_SAMPLES = 8192, 512
 SEED = 777
+
+
+DUMP_ROWS = 1 << 18      # arrays with more rows (first dimension) are dumped at this many fixed, seeded rows
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy: floating point as float32, integers / bools as float64 (exact).  A tensor with more
+    than DUMP_ROWS rows is written at DUMP_ROWS rows drawn with a fixed seed from its row count, so arrays of one length share rows
+    and two runs share positions.  Grids are flattened first.  Bounded at ~8 bytes x DUMP_ROWS x columns per array (~15 MB for
+    the truck step)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.dim() >= 4:
+            t = t.reshape(-1)
+        if t.dim() and t.shape[0] > DUMP_ROWS:
+            g = torch.Generator().manual_seed(SEED * 1000003 + t.shape[0])
+            idx = torch.randint(0, t.shape[0], (DUMP_ROWS,), generator=g).sort().values
+            t = t[idx.to(t.device)]
+        t = t.float() if t.is_floating_point() else t.double()
+        np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy())
+
+
+def step_arrays(ret, loss, model):
+    """The tensors of a forward's result dict, the loss and the parameters, named for dump_outputs."""
+    out = {k: v for k, v in ret.items() if torch.is_tensor(v)}
+    if loss is not None:
+        out['loss'] = loss
+    out.update({'param.' + k: v for k, v in model.named_parameters()})
+    return out
 
 
 def workload_kwargs(name):
@@ -338,6 +373,8 @@ def render_workload(args, emit):
     torch.cuda.synchronize()
     if world > 1:
         torch.distributed.barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_arrays(out if args.workload == 'garden' else {'rgb_marched': out[0]}, None, model))
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         torch.distributed.all_reduce(ms, op=torch.distributed.ReduceOp.MAX)
@@ -410,7 +447,13 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-reference-gpu', action='store_true', help='skip the reference-GPU baseline leg (oracle/_ref + ATen) of the N = 1 line')
     ap.add_argument('--only-timed', action='store_true', help='warm-up + timed region only (for ncu captures)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed to DIR/<name>.npy (see dump_outputs)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
 
     # fd 1 carries exactly one JSON line: native libraries (NCCL's "NCCL version ..." banner) write to stderr instead
@@ -426,7 +469,6 @@ def main():
             if int(os.environ.get('RANK', '0')) == 0:
                 emit({'impl': args.impl, 'unavailable': 'the reference arm is defined for the training workloads (truck / bicycle) only'})
             return
-        args.steps = min(args.steps, 5)
         return render_workload(args, emit)
     from unboundednerfpytorch_b200 import dist as ubdist
     rank = int(os.environ.get('RANK', '0'))
@@ -526,6 +568,7 @@ def main():
 
     tail_events = []
     survivors = [N_RAYS * N_SAMPLES]
+    last_step = []                    # (ret, loss) of the latest step, kept only for --dump-outputs
 
     def train_step(ro, rd, vd, target, it):
         ret = model(ro, rd, vd, global_step=it, is_train=True, **rk)
@@ -552,6 +595,8 @@ def main():
             ubdist.reduce_tv_step(opt, tv_terms)
         ev[1].record()
         tail_events.append(ev)
+        if args.dump_outputs:
+            last_step[:] = [ret, loss]
         return loss
 
     def sync_all():
@@ -595,6 +640,9 @@ def main():
     _cabi.reset_launch_count()
     del tail_events[:]
     ms_total = timed_region(dev_step, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_arrays(last_step[0], last_step[1], model))
+    del last_step[:]
     tail_ms = sum(a.elapsed_time(b) for a, b in tail_events) / max(len(tail_events), 1)   # all-reduce + TV + Adam per step
     launches = _cabi.launch_count()
     ktimes = _cabi.TIMER.summary()

@@ -64,22 +64,23 @@ def build_pair(name, dev, n_rays=8192, seed=777):
     return ours, p, batch, stepsize, flavor
 
 
-def _stat(a, b):
+def _stat(a, b, scale=None, n=None):
     """Error statistics of a (ours) against b (reference GPU path):
     rel_scale = max |a-b| / max|b|                       (rtol * scale criterion)
     rel_elem  = max |a-b| / |b| over elements with |b| >= 1 % of the scale     (per-element relative error away from zero)
-    frac_gt   = fraction of elements with |a-b| > 1e-5 * max(|b|, 1 % scale)."""
+    frac_gt   = fraction of elements with |a-b| > 1e-5 * max(|b|, 1 % scale).
+    scale, n: max |b| and the element count of the whole tensor when a and b are samples of it (n_sample elements)."""
     a, b = a.detach().float(), b.detach().float().reshape(a.shape)
     if a.numel() == 0:
         return dict(n=0, max_abs=0.0, scale=0.0, rel_scale=0.0, rel_elem=0.0, frac_gt=0.0)
-    scale = b.abs().max().item()
+    scale = b.abs().max().item() if scale is None else scale
     err = (a - b).abs()
     floor = 0.01 * scale if scale > 0 else 1.0
     big = b.abs() >= floor
     rel_elem = (err[big] / b.abs()[big]).max().item() if bool(big.any()) else 0.0
     frac = (err > RTOL * b.abs().clamp_min(floor)).float().mean().item()
-    return dict(n=a.numel(), max_abs=err.max().item(), scale=scale, rel_scale=err.max().item() / (scale if scale > 0 else 1.0),
-                rel_elem=rel_elem, frac_gt=frac)
+    return dict(n=a.numel() if n is None else n, n_sample=a.numel(), max_abs=err.max().item(), scale=scale,
+                rel_scale=err.max().item() / (scale if scale > 0 else 1.0), rel_elem=rel_elem, frac_gt=frac)
 
 
 def colour_branch_fp64(flavor, p, ref, vd, target, n_rays, chunk=1 << 19):
@@ -144,14 +145,16 @@ def density_scatter_fp64(p, pts_q, g_density_q, chunk=1 << 20):
     return kg.grad
 
 
-def _vs_truth(a, b, truth):
-    """Deviation of ours (a) and of the reference GPU path (b) from the fp64 yardstick, relative to max |truth|."""
+def _vs_truth(a, b, truth, scale=None, n=None):
+    """Deviation of ours (a) and of the reference GPU path (b) from the fp64 yardstick, relative to max |truth| (scale and n: of
+    the whole tensor, when a, b and truth are samples of it)."""
     t = truth.reshape(b.shape)
-    scale = t.abs().max().item() or 1.0
+    scale = (t.abs().max().item() if scale is None else scale) or 1.0
     ea, eb = (a.detach().double() - t).abs(), (b.detach().double() - t).abs()
     tol = RTOL * scale
     return dict(scale=scale, ours_max=ea.max().item() / scale, ref_max=eb.max().item() / scale,
-                ours_n_bad=int((ea > tol).sum()), ref_n_bad=int((eb > tol).sum()), n=a.numel())
+                ours_n_bad=int((ea > tol).sum()), ref_n_bad=int((eb > tol).sum()), n=a.numel() if n is None else n,
+                n_sample=a.numel())
 
 
 def compare(name, dev, n_rays=8192, backward=True, ext=None, truth=True):
@@ -214,3 +217,125 @@ def compare(name, dev, n_rays=8192, backward=True, ext=None, truth=True):
         out['refself k0.grid'] = _stat(p['k0_grid'].grad, first['k0.grid'])
         del ref2, first
     return out, ours, p
+
+
+# ---------------------------------------------------------------------------------------------------------------------------
+# The same comparison without the reference: record() keeps, per configuration, what compare() judges this library against --
+# the sample set (digests); every reference output and gradient at SAMPLE fixed positions (k0.grid at K0_SAMPLE) with the scale
+# of the whole tensor; the fp64 gradients at the first TRUTH_SAMPLE of those positions (as float32 differences from the
+# reference's value: fp64-exact to ~1e-15 at float32 size) with the reference's deviation from them on those positions and on
+# the whole tensor; the reference's run-to-run statistics on the whole tensors -- and compare_recorded() judges a run of this
+# library against that record with the statistics above, taken on the stored positions against whole-tensor scales and counts.
+SAMPLE = 256
+K0_SAMPLE = 16384         # resolves the k0.grid bar frac_gt <= 1e-3 (16 elements); at 1.3e-4 (measured, full tensor) ~2 are expected
+TRUTH_SAMPLE = 4096
+
+
+def _index(nm, shape):
+    from tests.util import sample_index
+    return sample_index(shape, K0_SAMPLE if nm == 'k0.grid' else SAMPLE)
+
+
+def _numel(shape):
+    n = 1
+    for s in shape:
+        n *= int(s)
+    return n
+
+
+def count_bar(st):
+    """Largest count of elements beyond 1e-5 of scale against fp64 (ours_n_bad) that passes the whole-tensor bar
+    `ours_n_bad <= max(16, 3 x the reference's count)`.  On n_sample uniformly drawn positions of n, a tensor with N such elements
+    shows a count of about Poisson(n_sample N / n): the bar is that mean for N = max(16, 3 x the reference's whole-tensor count)
+    plus four of its standard deviations plus one, so a library within the whole-tensor bar passes on all but ~1e-4 of position
+    draws, and one several times over it fails.  On a whole tensor (n_sample = n) it is the whole-tensor bar itself."""
+    n, k = st['n'], st.get('n_sample', st['n'])
+    lam = k / n * max(16, 3 * st.get('ref_n_bad_full', st['ref_n_bad']))
+    return lam if k >= n else lam + 4 * lam ** 0.5 + 1
+
+
+def record(name, dev, ext, n_rays=8192):
+    """Run the reference GPU path (ext = its CUDA extension) once and reduce it to a record for compare_recorded()."""
+    import bench
+    from oracle import cpu_ref
+    from tests.util import digest, sample_index, take
+    _, p, (ro, rd, vd, target), stepsize, flavor = build_pair(name, dev, n_rays)
+    ref = cpu_ref.model_forward(flavor, p, ro, rd, vd, stepsize, bg=1, rand_bkgd=False, render_depth=True, ext=ext,
+                                keep_intermediates=True)
+    rec = {'M_ref': int(ref['ray_id'].numel()), 'ray_id': digest(ref['ray_id']), 'step_id': digest(ref['step_id']), 'out': {},
+           'grad': {}, 'truth': {}}
+    for k in FLOAT_KEYS:
+        if k in ref:
+            t = ref[k].detach()
+            rec['out'][k] = dict(shape=tuple(t.shape), scale=t.abs().max().item(), sample=take(t, sample_index(t.shape, SAMPLE)))
+    loss_ref = bench.step_loss(ref, target, n_rays)
+    g_dq = torch.autograd.grad(loss_ref, ref['_density_q'], retain_graph=True)[0]
+    loss_ref.backward()
+    grads = {'density.grid': p['density_grid'].grad, 'k0.grid': p['k0_grid'].grad}
+    grads.update({'rgbnet.' + k: v.grad for k, v in p['rgbnet'].items()})
+    for nm, g in grads.items():
+        rec['grad'][nm] = dict(shape=tuple(g.shape), scale=g.abs().max().item(), sample=take(g, _index(nm, g.shape)))
+    grads64, rec['n_relu_ambiguous'] = colour_branch_fp64(flavor, p, ref, vd, target, n_rays)
+    grads64['density.grid'] = density_scatter_fp64(p, ref['_pts_q'], g_dq)
+    del g_dq
+    for nm, t in grads64.items():
+        idx = _index(nm, t.shape)[:TRUTH_SAMPLE]
+        b, tt = take(grads[nm], idx), take(t, idx)
+        st = _vs_truth(b, b, tt, t.abs().max().item())
+        full = _vs_truth(grads[nm], grads[nm], t)
+        rec['truth'][nm] = dict(scale=full['scale'], delta=(tt - b.double()).float(), ref_max=st['ref_max'], ref_n_bad=st['ref_n_bad'],
+                                ref_max_full=full['ref_max'], ref_n_bad_full=full['ref_n_bad'])
+    del grads64
+    first = {nm: grads[nm].detach().clone() for nm in ('density.grid', 'k0.grid')}
+    for k in ('density_grid', 'k0_grid'):
+        p[k].grad = None
+    ref2 = cpu_ref.model_forward(flavor, p, ro, rd, vd, stepsize, bg=1, rand_bkgd=False, render_depth=False, ext=ext)
+    bench.step_loss(ref2, target, n_rays).backward()
+    rec['refself density.grid'] = _stat(p['density_grid'].grad, first['density.grid'])
+    rec['refself k0.grid'] = _stat(p['k0_grid'].grad, first['k0.grid'])
+    return rec
+
+
+def compare_recorded(name, dev, rec, n_rays=8192):
+    """compare() of this library's fused path against a record(): the same keys, the statistics taken on the stored positions
+    ('n' = element count of the whole tensor, 'n_sample' = positions compared; 'truth' entries carry the reference's
+    whole-tensor ref_max_full / ref_n_bad_full for count_bar).  'flips' is None when the sample set differs (the record holds
+    its digest, not the samples)."""
+    import bench
+    from tests.util import digest, sample_index, take
+    ours, p, (ro, rd, vd, target), stepsize, flavor = build_pair(name, dev, n_rays)
+    del p
+    out = {'config': name, 'flavor': flavor}
+    rk = dict(near=0., far=1e9, bg=1, rand_bkgd=False, stepsize=stepsize, render_depth=True)
+    ret = ours(ro, rd, vd, global_step=None, is_train=False, **rk)
+    out['M'], out['M_ref'], out['n_max'] = int(ret['ray_id'].numel()), rec['M_ref'], int(ret['n_max'])
+    out['ray_id_equal'] = digest(ret['ray_id']) == rec['ray_id']
+    out['step_id_equal'] = digest(ret['step_id']) == rec['step_id']
+    out['flips'] = 0 if out['ray_id_equal'] and out['step_id_equal'] else None
+    for k, r in rec['out'].items():
+        if k in ret:
+            assert tuple(ret[k].shape) == r['shape'], f'{name} {k}: shape {tuple(ret[k].shape)} vs {r["shape"]}'
+            out[k] = _stat(take(ret[k], sample_index(r['shape'], SAMPLE)), r['sample'], r['scale'], _numel(r['shape']))
+    if out['flips'] is None:
+        return out, ours
+    ours.zero_grad(set_to_none=True)
+    bench.step_loss(ret, target, n_rays).backward()
+    names = {'density.grid': ours.density.grid, 'k0.grid': ours.k0.grid, 'rgbnet.W1': ours.rgbnet[0].weight,
+             'rgbnet.b1': ours.rgbnet[0].bias, 'rgbnet.W2': ours.rgbnet[2][0].weight, 'rgbnet.b2': ours.rgbnet[2][0].bias,
+             'rgbnet.W3': ours.rgbnet[3].weight, 'rgbnet.b3': ours.rgbnet[3].bias}
+    for nm, v in names.items():
+        r = rec['grad'][nm]
+        assert tuple(v.grad.shape) == r['shape'], f'{name} grad {nm}: shape {tuple(v.grad.shape)} vs {r["shape"]}'
+        n = _numel(r['shape'])
+        a = take(v.grad, _index(nm, r['shape']))
+        out['grad ' + nm] = _stat(a, r['sample'], r['scale'], n)
+        if nm in rec['truth']:
+            t = rec['truth'][nm]
+            k = t['delta'].numel()
+            b = r['sample'][:k]
+            st = _vs_truth(a[:k], b, b.double() + t['delta'].double(), t['scale'], n)
+            out['truth ' + nm] = dict(st, ref_max=t['ref_max'], ref_n_bad=t['ref_n_bad'], ref_max_full=t['ref_max_full'],
+                                      ref_n_bad_full=t['ref_n_bad_full'])
+    out['n_relu_ambiguous'] = rec['n_relu_ambiguous']
+    out['refself density.grid'], out['refself k0.grid'] = rec['refself density.grid'], rec['refself k0.grid']
+    return out, ours

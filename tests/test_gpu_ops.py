@@ -1,12 +1,12 @@
 """GPU parity tests of the drop-in ops (through the C ABI) against
   (1) the CPU oracle on identical seeded inputs,
-  (2) the reference's OWN CUDA extension built into oracle/_ref (bit-exact for index / mask outputs), when present,
+  (2) the reference's OWN CUDA extension on the same inputs (bit-exact), as recorded in tests/golden/ref_gpu.pkl.xz,
   (3) the golden fixtures recorded from the reference's Python.
 Tolerance: bit-exact for int / bool outputs; 1e-5 relative for fp32 (BASELINE.json north_star)."""
 import pytest
 import torch
 
-from tests.util import assert_close, assert_equal, load_golden, ref_cuda
+from tests.util import assert_close, assert_equal, assert_equal_ref, load_golden
 
 pytestmark = pytest.mark.gpu
 DEV = 'cuda:0'
@@ -50,12 +50,11 @@ def test_ray_aabb_and_counts(ops, oracle, n):
     st_c, dr_c = oracle.infer_ray_start_dir(ro, rd, tmin_c)
     st_g, dr_g = ops.infer_ray_start_dir(args_g[0], args_g[1], tmin_g)
     assert_close(st_g, st_c, what='start'); assert_close(dr_g, dr_c, what='dir')
-    ref = ref_cuda('render_utils_cuda')
-    a, b = ref.infer_t_minmax(*args_g, 0.2, 1e9)
-    assert_equal(tmin_g, a, 't_min vs ref-cuda'); assert_equal(tmax_g, b, 't_max vs ref-cuda')
-    assert_equal(ns_g, ref.infer_n_samples(args_g[1], a, b, 0.03), 'N_steps vs ref-cuda')
-    a, b = ref.infer_ray_start_dir(args_g[0], args_g[1], tmin_g)
-    assert_equal(st_g, a, 'start vs ref-cuda'); assert_equal(dr_g, b, 'dir vs ref-cuda')
+    ru = lambda ref: ref('render_utils_cuda')
+    assert_equal_ref(f'infer_t_minmax/{n}', (tmin_g, tmax_g), lambda ref: ru(ref).infer_t_minmax(*args_g, 0.2, 1e9))
+    assert_equal_ref(f'infer_n_samples/{n}', ns_g,
+                     lambda ref: ru(ref).infer_n_samples(args_g[1], *ru(ref).infer_t_minmax(*args_g, 0.2, 1e9), 0.03))
+    assert_equal_ref(f'infer_ray_start_dir/{n}', (st_g, dr_g), lambda ref: ru(ref).infer_ray_start_dir(args_g[0], args_g[1], tmin_g))
 
 
 @pytest.mark.parametrize('n', [1, 33, 1024, 8192])
@@ -64,10 +63,9 @@ def test_sample_pts_on_rays(ops, oracle, n):
     mn, mx = BOX
     stepdist = 0.5 * 2 / 64
     out_g = ops.sample_pts_on_rays(ro.to(DEV), rd.to(DEV), mn.to(DEV), mx.to(DEV), 0.2, 1e9, stepdist)
-    ref = ref_cuda('render_utils_cuda')
-    out_r = ref.sample_pts_on_rays(ro.to(DEV), rd.to(DEV), mn.to(DEV), mx.to(DEV), 0.2, 1e9, stepdist)
-    for a, b, nm in zip(out_g, out_r, ('pts', 'mask_outbbox', 'ray_id', 'step_id', 'N_steps', 't_min', 't_max')):
-        assert_equal(a, b, nm + ' vs ref-cuda')         # floats too: same arithmetic, same compiler
+    # floats too: same arithmetic, same compiler
+    assert_equal_ref(f'sample_pts_on_rays/{n}', out_g, lambda ref: ref('render_utils_cuda').sample_pts_on_rays(
+        ro.to(DEV), rd.to(DEV), mn.to(DEV), mx.to(DEV), 0.2, 1e9, stepdist))
     out_c = oracle.sample_pts_on_rays(ro, rd, mn, mx, 0.2, 1e9, stepdist)
     if torch.equal(out_g[4].cpu(), out_c[4]):
         for a, b, nm in zip(out_g, out_c, ('pts', 'mask_outbbox', 'ray_id', 'step_id', 'N_steps', 't_min', 't_max')):
@@ -92,14 +90,14 @@ def test_sample_ndc_and_bg(ops, oracle):
     pg, mg = ops.sample_ndc_pts_on_rays(ro.to(DEV), rd.to(DEV), mn.to(DEV), mx.to(DEV), 65)
     pc, mc = oracle.sample_ndc_pts_on_rays(ro, rd, mn, mx, 65)
     assert_close(pg, pc, what='ndc pts'); assert (mg.cpu() != mc).float().mean() < 1e-4
-    tmax = torch.rand(257) + 1
+    tmax = torch.rand(257, generator=torch.Generator().manual_seed(6)) + 1
     bg = ops.sample_bg_pts_on_rays(ro.to(DEV), rd.to(DEV), tmax.to(DEV), 0.5, 32)
     bc = oracle.sample_bg_pts_on_rays(ro, rd, tmax, 0.5, 32)
     assert_close(bg, bc, rtol=2e-5, what='bg pts')
-    ref = ref_cuda('render_utils_cuda')
-    pr, mr = ref.sample_ndc_pts_on_rays(ro.to(DEV), rd.to(DEV), mn.to(DEV), mx.to(DEV), 65)
-    assert_equal(pg, pr, 'ndc pts vs ref-cuda'); assert_equal(mg, mr, 'ndc mask vs ref-cuda')
-    assert_equal(bg, ref.sample_bg_pts_on_rays(ro.to(DEV), rd.to(DEV), tmax.to(DEV), 0.5, 32), 'bg vs ref-cuda')
+    assert_equal_ref('sample_ndc_pts_on_rays', (pg, mg), lambda ref: ref('render_utils_cuda').sample_ndc_pts_on_rays(
+        ro.to(DEV), rd.to(DEV), mn.to(DEV), mx.to(DEV), 65))
+    assert_equal_ref('sample_bg_pts_on_rays', bg, lambda ref: ref('render_utils_cuda').sample_bg_pts_on_rays(
+        ro.to(DEV), rd.to(DEV), tmax.to(DEV), 0.5, 32))
 
 
 @pytest.mark.parametrize('n', [0, 1, 999, 300000])
@@ -114,9 +112,9 @@ def test_maskcache_lookup(ops, oracle, n):
     out_c = oracle.maskcache_lookup(mask, xyz, scale, shift)
     assert out_g.dtype == torch.bool and out_g.shape == (n,)
     assert_equal(out_g, out_c, 'maskcache vs oracle')           # same fma + round-half-away => bit exact
-    ref = ref_cuda('render_utils_cuda')
     if n > 0:
-        assert_equal(out_g, ref.maskcache_lookup(mask.to(DEV), xyz.to(DEV), scale.to(DEV), shift.to(DEV)), 'vs ref-cuda')
+        assert_equal_ref(f'maskcache_lookup/{n}', out_g, lambda ref: ref('render_utils_cuda').maskcache_lookup(
+            mask.to(DEV), xyz.to(DEV), scale.to(DEV), shift.to(DEV)))
 
 
 def test_maskgrid_golden():
@@ -149,11 +147,11 @@ def test_raw2alpha(ops, oracle, n):
     assert_close(a2, a2c, what='alpha nonuni')
     assert_close(ops.raw2alpha_nonuni_backward(e2, gb.to(DEV), itv.to(DEV))[fin.to(DEV)],
                  oracle.raw2alpha_nonuni_backward(e2c, gb, itv)[fin], what='nonuni grad')
-    ref = ref_cuda('render_utils_cuda')
     if n > 0:
-        er, ar = ref.raw2alpha(d.to(DEV), -2.0, 0.5)
-        assert_equal(a_g, ar, 'alpha vs ref-cuda'); assert_equal(e_g, er, 'exp vs ref-cuda')
-        assert_equal(g_g, ref.raw2alpha_backward(er, gb.to(DEV), 0.5), 'grad vs ref-cuda')
+        ru = lambda ref: ref('render_utils_cuda')
+        assert_equal_ref(f'raw2alpha/{n}', (e_g, a_g), lambda ref: ru(ref).raw2alpha(d.to(DEV), -2.0, 0.5))
+        assert_equal_ref(f'raw2alpha_backward/{n}', g_g,
+                         lambda ref: ru(ref).raw2alpha_backward(ru(ref).raw2alpha(d.to(DEV), -2.0, 0.5)[0], gb.to(DEV), 0.5))
 
 
 def _ragged(n_rays, max_len, seed, opaque_frac=0.3):
@@ -180,12 +178,12 @@ def test_alpha2weight_ragged(ops, oracle, n_rays, max_len):
     gg = ops.alpha2weight_backward(alpha.to(DEV), *out_g, n_rays, gw.to(DEV), gl.to(DEV))
     gc = oracle.alpha2weight_backward(alpha, *out_c, n_rays, gw, gl)
     assert_close(gg, gc, rtol=2e-5, atol=1e-6, what='alpha2weight grad')
-    ref = ref_cuda('render_utils_cuda')
     if len(alpha) > 0:
-        out_r = ref.alpha2weight(alpha.to(DEV), ray_id.to(DEV), n_rays)
-        for a, b, nm in zip(out_g, out_r, names):
-            assert_equal(a, b, nm + ' vs ref-cuda')
-        assert_equal(gg, ref.alpha2weight_backward(alpha.to(DEV), *out_r, n_rays, gw.to(DEV), gl.to(DEV)), 'grad vs ref-cuda')
+        ru = lambda ref: ref('render_utils_cuda')
+        key = f'alpha2weight/{n_rays}-{max_len}'
+        assert_equal_ref(key, out_g, lambda ref: ru(ref).alpha2weight(alpha.to(DEV), ray_id.to(DEV), n_rays))
+        assert_equal_ref(key + '/backward', gg, lambda ref: ru(ref).alpha2weight_backward(
+            alpha.to(DEV), *ru(ref).alpha2weight(alpha.to(DEV), ray_id.to(DEV), n_rays), n_rays, gw.to(DEV), gl.to(DEV)))
 
 
 def test_alpha2weight_full_size_properties(ops):
@@ -238,8 +236,8 @@ def test_cumdist_thres(ops, oracle, n_rays, n_pts):
     dist = torch.rand(n_rays, n_pts, generator=g) * 0.02
     out_g = ops.cumdist_thres(dist.to(DEV), 0.0149)
     assert_equal(out_g, oracle.cumdist_thres(dist, 0.0149), 'cumdist vs oracle')     # same sequential float adds
-    ref = ref_cuda('ub360_utils_cuda')
-    assert_equal(out_g, ref.cumdist_thres(dist.to(DEV), 0.0149), 'cumdist vs ref-cuda')
+    assert_equal_ref(f'cumdist_thres/{n_rays}-{n_pts}', out_g,
+                     lambda ref: ref('ub360_utils_cuda').cumdist_thres(dist.to(DEV), 0.0149))
 
 
 @pytest.mark.parametrize('shape,layout', [((1, 1, 5, 6, 7), 'ref'), ((1, 12, 9, 8, 10), 'ref'), ((9, 12, 6, 5, 7), 'cl'),
@@ -260,10 +258,12 @@ def test_total_variation(ops, oracle, shape, layout):
         assert_close(g_g, grad_c, what=f'tv dense={dense}')
         if not dense:
             assert torch.equal(g_g.cpu()[grad == 0], grad[grad == 0])        # untouched where grad was 0
-        ref = ref_cuda('total_variation_cuda')
-        g_r = grad.to(DEV)
-        ref.total_variation_add_grad(param.to(DEV), g_r, 0.3, 0.2, 0.1, dense)
-        assert_equal(g_g.contiguous(), g_r, 'tv vs ref-cuda')
+
+        def tv_ref(ref):
+            g_r = grad.to(DEV)
+            ref('total_variation_cuda').total_variation_add_grad(param.to(DEV), g_r, 0.3, 0.2, 0.1, dense)
+            return g_r
+        assert_equal_ref(f'total_variation_add_grad/{"x".join(map(str, shape))}/{layout}/{int(dense)}', g_g.contiguous(), tv_ref)
     tv = load_golden('l1_grids.pt')['tv']
     for k in ('dense1', 'dense0'):
         gg = tv[k]['grad_in'].to(DEV)
@@ -278,23 +278,29 @@ def test_adam_variants(ops, oracle, n):
         p = torch.randn(n, generator=g); m = torch.zeros(n); v = torch.zeros(n)
         perlr = torch.rand(n, generator=g)
         pg, mg, vg, lg = p.to(DEV), m.to(DEV), v.to(DEV), perlr.to(DEV)
-        refm = ref_cuda('adam_upd_cuda')
-        pr, mr, vr = pg.clone(), mg.clone(), vg.clone()
+        pr, mr, vr = pg.clone(), mg.clone(), vg.clone()          # the reference's state (advanced while recording)
         for step in (1, 2, 3):
             grad = torch.randn(n, generator=g) * (torch.rand(n, generator=g) > 0.5)
             gg = grad.to(DEV)
             if mode == 0:
                 oracle.adam_upd(p, grad, m, v, step, 0.9, 0.99, 0.1, 1e-8); ops.adam_upd(pg, gg, mg, vg, step, 0.9, 0.99, 0.1, 1e-8)
-                refm.adam_upd(pr, gg, mr, vr, step, 0.9, 0.99, 0.1, 1e-8)
             elif mode == 1:
                 oracle.masked_adam_upd(p, grad, m, v, step, 0.9, 0.99, 0.1, 1e-8); ops.masked_adam_upd(pg, gg, mg, vg, step, 0.9, 0.99, 0.1, 1e-8)
-                refm.masked_adam_upd(pr, gg, mr, vr, step, 0.9, 0.99, 0.1, 1e-8)
             else:
                 oracle.adam_upd_with_perlr(p, grad, m, v, perlr, step, 0.9, 0.99, 0.1, 1e-8)
                 ops.adam_upd_with_perlr(pg, gg, mg, vg, lg, step, 0.9, 0.99, 0.1, 1e-8)
-                refm.adam_upd_with_perlr(pr, gg, mr, vr, lg, step, 0.9, 0.99, 0.1, 1e-8)
             assert_close(pg, p, what=f'adam mode {mode} p'); assert_close(mg, m, what='m'); assert_close(vg, v, what='v')
-            assert_equal(pg, pr, f'adam mode {mode} p vs ref-cuda'); assert_equal(mg, mr, 'm vs ref-cuda'); assert_equal(vg, vr, 'v vs ref-cuda')
+
+            def adam_ref(ref, gg=gg, step=step):
+                refm = ref('adam_upd_cuda')
+                if mode == 0:
+                    refm.adam_upd(pr, gg, mr, vr, step, 0.9, 0.99, 0.1, 1e-8)
+                elif mode == 1:
+                    refm.masked_adam_upd(pr, gg, mr, vr, step, 0.9, 0.99, 0.1, 1e-8)
+                else:
+                    refm.adam_upd_with_perlr(pr, gg, mr, vr, lg, step, 0.9, 0.99, 0.1, 1e-8)
+                return pr, mr, vr
+            assert_equal_ref(f'adam/{n}/mode{mode}/step{step}', (pg, mg, vg), adam_ref)
 
 
 def test_masked_adam_golden_and_fused_tail(ops):
